@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — MPC solves/sec of the batched update -> solve -> output step (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload identical|random]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload identical|random] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -16,6 +16,9 @@ Multi-GPU: batch sharded over ranks (weak scaling, 65 536 instances per GPU); u*
 gathered buffer (peer stores fused into the solver epilogue + one arrival-flag kernel, or one NCCL all-gather with
 --nccl-gather); the gathered buffer is verified against an NCCL all-gather after the timed loop.
 The oracle (oracle/) is used ONLY for the cpu_baseline leg, the spot checks and --impl reference.
+--dump-outputs DIR: after the run, DIR/u.npy holds u* [global batch, nu] (float64) of the last timed step of the device-resident loop
+and DIR/u_e2e.npy that of the end-to-end loop (--impl reference: DIR/u.npy of the last timed CPU step).  The inputs are seeded, so
+runs with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -29,6 +32,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the tree it runs from
 
 B_PER_GPU = 65536
 ALG_BYTES_PER_ITER = 24 * (188 + 2 * 209)     # SURVEY.md §8d: 24 (n + 2 m) on the reference QP dims = 14 544 B
@@ -51,6 +55,12 @@ def mimo_batch(B, seed=4):
     from pympc_b200.workloads import mimo
     cfg = mimo(); rng = np.random.default_rng(seed)
     return cfg, np.ascontiguousarray(0.3 * rng.standard_normal((B, 8))), np.ascontiguousarray(np.tile(cfg["xref"], (B, 1)))
+
+
+def dump_outputs(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def load_json(*path):
@@ -150,7 +160,7 @@ def cpu_arm(steps, warmup, sample_b, workload, threads=None, **settings):
         U = Un; X = X @ Ad.T + U @ Bd.T
     bc.close()
     tot = float(np.sum(times))
-    return {"value": sample_b * steps / tot, "unit": UNIT, "cores": int(threads), "kind": "port",
+    return {"u": Un, "value": sample_b * steps / tot, "unit": UNIT, "cores": int(threads), "kind": "port",
             "sample": f"{sample_b} pendulum instances x {steps} closed-loop steps ({workload}), OSQP-port eps={settings.get('eps_abs', 1e-3):g}, "
                       f"mean {np.mean(iters):.0f} ADMM its/solve, solver-only (no Python per-instance overhead)",
             "ms_per_step": 1e3 * tot / steps}
@@ -437,15 +447,20 @@ def gpu_arm(args, rank, world, local_rank):
     sampler = ClockSampler(local_rank) if rank == 0 else None
     tot_ms_max, acc, rounds, Xd = device_loop(torch, dist, K, cfgp, X0, args.steps, args.warmup, dev, world, G, flush, sampler)
     clocks = sampler.stop() if rank == 0 else None
+    dumped = {"u": G.gathered().cpu().numpy()} if args.dump_outputs else None
     gather_ok = G.verify()
     # ---- end-to-end through the public API with pinned host buffers (H2D and D2H inside the timed region)
     e2e_t, Xh, Uh = e2e_loop(torch, dist, K, cfgp, X0, args.steps, args.warmup, dev, world, G, flush)
     gather_ok_e2e = G.verify()
+    if dumped is not None:
+        dumped["u_e2e"] = G.gathered().cpu().numpy() if world > 1 else Uh
     if world > 1 and not (gather_ok and gather_ok_e2e):
         raise SystemExit(f"rank {rank}: gathered u* buffer differs from the NCCL all-gather of the ranks' outputs")
     K.close()
     if rank != 0:
         return None
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped)
     peaks = load_json("MEASURED_PEAKS.json")
     shape_key = "pendulum_4_1_20_20"
     kern, peak_tf, hbm = roofline_entries(shape_key, acc, args.steps, peaks)
@@ -524,6 +539,7 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the configs[2] / configs[3] side measurements")
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"], help="strong: 524 288 instances in total (configs[4])")
     ap.add_argument("--nccl-gather", action="store_true", help="use the NCCL all-gather instead of fused peer stores")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write u* of the last timed step to DIR/*.npy")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3
@@ -534,6 +550,8 @@ def main():
         if rank != 0:
             return
         cb = cpu_arm(args.steps, args.warmup, args.cpu_sample, args.workload)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"u": cb["u"]})
         line = {"impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": args.gpus,
                 "steps": args.steps, "warmup": args.warmup, "ms_per_step": cb["ms_per_step"], "higher_is_better": True,
                 "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic",

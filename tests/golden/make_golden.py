@@ -1,25 +1,30 @@
-"""Generates the committed golden fixtures (run HERE, where /root/reference exists).
+"""Generates the committed golden fixtures from a checkout of the reference, forgi86/pyMPC.
 
 For every case the QP is assembled by the UNMODIFIED reference (pyMPC.mpc.MPCController with a
 stub ``osqp`` module, tests/refharness.py), solved by ``oracle.kkt.solve_exact`` and certified by
 the solver-independent KKT residuals (< 1e-9) on the reference-assembled (P, q, A, l, u).
 Closed loops use the linear plant x+ = Ad x + Bd u (README.md:59-77 pattern).
+ref_assembly.npz and pend_osqp_calls.npz hold what the reference itself computed and handed to
+its solver, so that the tests compare against the reference without needing it.
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py PATH_TO_PYMPC_CHECKOUT [fixture ...]
 """
+import json
 import os
 import sys
 
 import numpy as np
+import scipy.sparse as sp
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 from refharness import load_reference_controller  # noqa: E402
 from oracle.kkt import solve_exact, kkt_residuals  # noqa: E402
 from pympc_b200.workloads import point_mass, pendulum, mimo, pendulum_random  # noqa: E402
+from test_oracle import LIVE_VARIANTS, live_variant  # noqa: E402
 
 OUT = os.path.dirname(os.path.abspath(__file__))
-MPC = load_reference_controller()
+MPC = None
 
 
 def exact(K, warm=None):
@@ -98,10 +103,65 @@ def variants():
     print("variants ok")
 
 
+def put_csc(out, name, M):
+    M = sp.csc_matrix(M)
+    out[name + "_data"], out[name + "_indices"], out[name + "_indptr"], out[name + "_shape"] = M.data, M.indices, M.indptr, np.array(M.shape)
+
+
+def reference_assembly():
+    """the reference's (P, A, q, l, u) at setup and (q, l, u, J_CNST) after three updates with seeded random x, u_-1, xref, for
+    every case of tests/test_oracle.py::test_assembly_matches_reference_live"""
+    out = {}
+    for v in LIVE_VARIANTS:
+        cfg = live_variant(v)
+        K = MPC(**cfg); K.setup(solve=False)
+        put_csc(out, f"{v}__P", K.P); put_csc(out, f"{v}__A", K.A)
+        out[f"{v}__q"], out[f"{v}__l"], out[f"{v}__u"] = K.q.copy(), K.l.copy(), K.u.copy()
+        rng = np.random.default_rng(3); rec = {k: [] for k in ("x", "um1", "xref", "q", "l", "u", "J_CNST")}
+        for t in range(3):
+            x = rng.normal(size=K.nx); um1 = rng.normal(size=K.nu)
+            xr = np.array(cfg["xref"]) if t == 0 else rng.normal(size=np.shape(cfg["xref"]))
+            K.update(x, um1, xref=xr, solve=False)
+            for k, val in (("x", x), ("um1", um1), ("xref", xr), ("q", K.q), ("l", K.l), ("u", K.u), ("J_CNST", K.J_CNST)):
+                rec[k].append(np.copy(val))
+        for k, vals in rec.items():
+            out[f"{v}__upd_{k}"] = np.array(vals)
+    np.savez_compressed(os.path.join(OUT, "ref_assembly.npz"), **out)
+    print("ref_assembly", len(out), "arrays")
+
+
+def pend_osqp_calls(nsteps=5):
+    """what the reference hands its `osqp` object in the pendulum closed loop at eps 1e-9: the setup() call (matrices, vectors,
+    keyword arguments), then the update(l=, u=, q=) of each step, the states and previous inputs taken from pend_loop.npz"""
+    cfg = pendulum(); g = np.load(os.path.join(OUT, "pend_loop.npz"))
+    K = MPC(**cfg, eps_abs=1e-9, eps_rel=1e-9); K.setup(solve=False)
+    (P, q, A, l, u), kw = K.prob.setup_args
+    out = {"q": np.copy(q), "l": np.copy(l), "u": np.copy(u), "setup_kwargs": np.array(json.dumps(kw, sort_keys=True))}
+    put_csc(out, "P", P); put_csc(out, "A", A)
+    rec = {"q": [], "l": [], "u": []}
+    for t in range(nsteps):
+        um1 = np.array(cfg["uminus1"], float) if t == 0 else g["u"][t - 1]
+        K.update(g["x"][t], um1, solve=False)
+        for k in rec:
+            rec[k].append(np.copy(K.prob.update_args[k]))
+    for k, vals in rec.items():
+        out["upd_" + k] = np.array(vals)
+    np.savez_compressed(os.path.join(OUT, "pend_osqp_calls.npz"), **out)
+    print("pend_osqp_calls", kw)
+
+
+FIXTURES = {
+    "pm_first": lambda: first_solve("pm", point_mass()), "pend_first": lambda: first_solve("pend", pendulum()),
+    "mimo_first": lambda: first_solve("mimo", mimo()),
+    "pm_loop": lambda: closed_loop("pm", point_mass(), 30), "pend_loop": lambda: closed_loop("pend", pendulum(), 40),
+    "mimo_loop": lambda: closed_loop("mimo", mimo(), 12),
+    "pend_rand": random_batch, "variants": variants, "ref_assembly": reference_assembly, "pend_osqp_calls": pend_osqp_calls,
+}
+
+
 if __name__ == "__main__":
-    first_solve("pm", point_mass()); first_solve("pend", pendulum()); first_solve("mimo", mimo())
-    closed_loop("pm", point_mass(), 30)
-    closed_loop("pend", pendulum(), 40)
-    closed_loop("mimo", mimo(), 12)
-    random_batch()
-    variants()
+    if len(sys.argv) < 2:
+        raise SystemExit(__doc__)
+    MPC = load_reference_controller(os.path.abspath(sys.argv[1]))
+    for name in sys.argv[2:] or FIXTURES:
+        FIXTURES[name]()

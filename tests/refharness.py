@@ -1,20 +1,15 @@
-"""Loads the UNMODIFIED reference (``/root/reference/pyMPC/mpc.py``) with a stub ``osqp`` module.
+"""Loads the UNMODIFIED reference (``pyMPC/mpc.py`` of a forgi86/pyMPC checkout) with a stub ``osqp`` module.
 
-Only usable where /root/reference exists (this container, not the GPU box): used by
-``tests/golden/make_golden.py`` to generate committed fixtures and by tests that skip otherwise.
-The stub records what pyMPC hands to the solver (SURVEY.md Appendix C)."""
+Used only by ``tests/golden/make_golden.py`` to generate the committed fixtures; the tests themselves read the fixtures and
+never need the reference.  The stub records what pyMPC hands to the solver (SURVEY.md Appendix C)."""
 import os
 import sys
 import types
 
-REFERENCE_ROOT = "/root/reference"
 
-
-def reference_available():
-    return os.path.isfile(os.path.join(REFERENCE_ROOT, "pyMPC", "mpc.py"))
-
-
-def load_reference_controller():
+def load_reference_controller(reference_root):
+    if not os.path.isfile(os.path.join(reference_root, "pyMPC", "mpc.py")):
+        raise FileNotFoundError(f"{reference_root} is not a pyMPC checkout (no pyMPC/mpc.py)")
     if "osqp" not in sys.modules:
         stub = types.ModuleType("osqp")
 
@@ -31,7 +26,7 @@ def load_reference_controller():
         stub.OSQP = _OSQP
         stub.__stub__ = True
         sys.modules["osqp"] = stub
-    if REFERENCE_ROOT not in sys.path:
-        sys.path.insert(0, REFERENCE_ROOT)
+    if reference_root not in sys.path:
+        sys.path.insert(0, reference_root)
     from pyMPC.mpc import MPCController
     return MPCController

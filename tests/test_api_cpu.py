@@ -37,12 +37,18 @@ def test_create_argument_errors(bmpc_lib):
 
 
 def test_no_cpu_fallback_without_device(bmpc_lib):
-    if bmpc_lib.bmpc_device_count() > 0:
-        pytest.skip("a GPU is visible here")
-    from pympc_b200 import MPCController, BmpcError
-    K = MPCController(**point_mass())
-    with pytest.raises(BmpcError, match="no CUDA device"):
-        K.setup()
+    """in a process that sees no device (CUDA_VISIBLE_DEVICES empty, so this runs on GPU machines too), setup() raises"""
+    import subprocess, sys
+    code = ("import sys; sys.path.insert(0, sys.argv[1])\n"
+            "from pympc_b200 import MPCController, BmpcError, _lib\n"
+            "from pympc_b200.workloads import point_mass\n"
+            "assert _lib.load().bmpc_device_count() == 0\n"
+            "K = MPCController(**point_mass())\n"
+            "try:\n    K.setup()\nexcept BmpcError as exc:\n    print(exc)\nelse:\n    raise SystemExit('setup() succeeded without a device')\n")
+    r = subprocess.run([sys.executable, "-c", code, ROOT], capture_output=True, text=True, timeout=300,
+                       env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+    assert r.returncode == 0, r.stdout + r.stderr
+    assert re.search("no CUDA device", r.stdout), r.stdout
 
 
 @pytest.mark.parametrize("kw,msg", [

@@ -1,15 +1,36 @@
 """CPU tests of the oracle: assembly vs the reference / golden fixtures, exact solver and the C
 restatement of OSQP vs the KKT-certified goldens."""
+import json
+
 import numpy as np
 import pytest
+import scipy.sparse as sp
 
 from conftest import golden
 from oracle.qp_assembly import QPData
 from oracle.kkt import solve_exact, kkt_residuals
 from pympc_b200.workloads import point_mass, pendulum, mimo, WORKLOADS
-from refharness import reference_available, load_reference_controller
 
 CASES = {"pm": point_mass, "pend": pendulum, "mimo": mimo}
+LIVE_VARIANTS = ["pm", "pend", "mimo", "pm_Nc_tv", "mimo_Nc_uref", "pend_inf"]
+
+
+def live_variant(variant):
+    """configuration of one case of test_assembly_matches_reference_live (also read by tests/golden/make_golden.py)"""
+    if variant in CASES:
+        return CASES[variant]()
+    if variant == "pm_Nc_tv":
+        cfg = point_mass(); cfg["Np"] = 25; cfg["Nc"] = 10; cfg["xref"] = np.kron(np.ones((26, 1)), cfg["xref"])
+    elif variant == "mimo_Nc_uref":
+        cfg = mimo(); cfg["Np"] = 12; cfg["Nc"] = 5; cfg["uref"] = np.array([0.1, -0.2, 0.3, 0.0]); cfg["Qu"] = np.diag([1., 2, 3, 4])
+    else:
+        cfg = pendulum(); cfg["Qx"] = sp.diags([0.3, 0, 1.0, 0]); cfg["xmax"] = np.array([np.inf, 1, 2, 3]); cfg["Dumin"] = np.array([-np.inf])
+    return cfg
+
+
+def golden_csc(g, name):
+    """a sparse matrix stored by tests/golden/make_golden.py as its CSC arrays"""
+    return sp.csc_matrix((g[name + "_data"], g[name + "_indices"], g[name + "_indptr"]), shape=tuple(g[name + "_shape"]))
 
 
 @pytest.mark.parametrize("name", list(CASES))
@@ -25,31 +46,21 @@ def test_assembly_matches_golden_vectors(name):
     assert np.allclose([Q.A.sum(), np.abs(Q.A).sum()], g["A_sum"], rtol=0, atol=1e-12)
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference not present on this box")
-@pytest.mark.parametrize("variant", ["pm", "pend", "mimo", "pm_Nc_tv", "mimo_Nc_uref", "pend_inf"])
+@pytest.mark.parametrize("variant", LIVE_VARIANTS)
 def test_assembly_matches_reference_live(variant):
-    MPC = load_reference_controller()
-    import scipy.sparse as sp
-    if variant in CASES:
-        cfg = CASES[variant]()
-    elif variant == "pm_Nc_tv":
-        cfg = point_mass(); cfg["Np"] = 25; cfg["Nc"] = 10; cfg["xref"] = np.kron(np.ones((26, 1)), cfg["xref"])
-    elif variant == "mimo_Nc_uref":
-        cfg = mimo(); cfg["Np"] = 12; cfg["Nc"] = 5; cfg["uref"] = np.array([0.1, -0.2, 0.3, 0.0]); cfg["Qu"] = np.diag([1., 2, 3, 4])
-    else:
-        cfg = pendulum(); cfg["Qx"] = sp.diags([0.3, 0, 1.0, 0]); cfg["xmax"] = np.array([np.inf, 1, 2, 3]); cfg["Dumin"] = np.array([-np.inf])
-    K = MPC(**cfg); K.setup(solve=False)
+    """(P, A, q, l, u) and J_CNST exactly as the unmodified reference's MPCController assembled them, at setup and after three
+    update() calls with random x, u_-1 and xref (stored by tests/golden/make_golden.py in ref_assembly.npz)"""
+    g = golden("ref_assembly.npz")
+    k = lambda name: g[f"{variant}__{name}"]
+    cfg = live_variant(variant)
     Q = QPData(**cfg)
     fin = lambda v: np.where(np.isinf(v), 0, v)
-    assert np.array_equal(K.P.toarray(), Q.P) and np.array_equal(K.A.toarray(), Q.A)
-    assert np.array_equal(K.q, Q.q) and np.array_equal(fin(K.l), fin(Q.l)) and np.array_equal(fin(K.u), fin(Q.u))
-    rng = np.random.default_rng(3)
+    assert np.array_equal(golden_csc(g, f"{variant}__P").toarray(), Q.P) and np.array_equal(golden_csc(g, f"{variant}__A").toarray(), Q.A)
+    assert np.array_equal(k("q"), Q.q) and np.array_equal(fin(k("l")), fin(Q.l)) and np.array_equal(fin(k("u")), fin(Q.u))
     for t in range(3):
-        x = rng.normal(size=Q.nx); um1 = rng.normal(size=Q.nu)
-        xr = cfg["xref"] if t == 0 else rng.normal(size=np.shape(cfg["xref"]))
-        K.update(x, um1, xref=xr, solve=False); Q.update(x, um1, xr)
-        assert np.array_equal(K.q, Q.q) and np.array_equal(fin(K.l), fin(Q.l)) and np.array_equal(fin(K.u), fin(Q.u))
-        assert abs(K.J_CNST - Q.constant_term()) < 1e-12
+        Q.update(k("upd_x")[t], k("upd_um1")[t], k("upd_xref")[t])
+        assert np.array_equal(k("upd_q")[t], Q.q) and np.array_equal(fin(k("upd_l")[t]), fin(Q.l)) and np.array_equal(fin(k("upd_u")[t]), fin(Q.u))
+        assert abs(k("upd_J_CNST")[t] - Q.constant_term()) < 1e-12
 
 
 @pytest.mark.parametrize("name", ["pm", "pend"])
@@ -87,37 +98,26 @@ def test_osqp_port_default_and_tight(name, osqp_port_lib):
     assert abs(r2.info.obj_val - float(g["obj"])) < 1e-6 * (1 + abs(float(g["obj"])))
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference not present on this box")
 def test_unmodified_reference_runs_on_the_port(osqp_port_lib):
-    """Reference MPCController end to end with osqp_port injected as `osqp` (tight tolerance) vs golden loop."""
-    import sys
-    saved = sys.modules.get("osqp")
-    sys.modules["osqp"] = osqp_port_lib
-    try:
-        for m in [k for k in sys.modules if k.startswith("pyMPC")]:
-            del sys.modules[m]
-        sys.path.insert(0, "/root/reference")
-        from pyMPC.mpc import MPCController
-        cfg = pendulum()
-        K = MPCController(**cfg, eps_abs=1e-9, eps_rel=1e-9)
-        K.setup(solve=False)
-        # the reference does not forward max_iter; tight tolerance needs more than OSQP's 4000 default
-        K.prob = osqp_port_lib.OSQP()
-        K.prob.setup(K.P, K.q, K.A, K.l, K.u, warm_start=True, eps_abs=1e-9, eps_rel=1e-9, max_iter=200000)
-        K.solve()
-        g = golden("pend_loop.npz")
-        x = np.array(cfg["x0"]); um1 = np.array(cfg["uminus1"])
-        for t in range(5):
-            K.update(x, um1); u = np.array(K.output())
-            assert np.max(np.abs(u - g["u"][t])) < 1e-6
-            x = cfg["Ad"] @ x + cfg["Bd"] @ u; um1 = u
-    finally:
-        for m in [k for k in sys.modules if k.startswith("pyMPC")]:
-            del sys.modules[m]
-        if saved is not None:
-            sys.modules["osqp"] = saved
-        else:
-            sys.modules.pop("osqp", None)
+    """The calls the unmodified reference MPCController makes on its `osqp` object in the pendulum closed loop (eps 1e-9),
+    recorded along the golden loop's states by tests/golden/make_golden.py in pend_osqp_calls.npz, replayed on osqp_port:
+    setup() with the reference's own keyword arguments, then per step update(l=, u=, q=) and solve(), read back the way
+    output() does (status, res.x slice), against the golden loop."""
+    c = golden("pend_osqp_calls.npz"); g = golden("pend_loop.npz")
+    P, A = golden_csc(c, "P"), golden_csc(c, "A")
+    kw = json.loads(str(c["setup_kwargs"]))
+    osqp_port_lib.OSQP().setup(P, c["q"], A, c["l"], c["u"], **kw)
+    # the reference does not forward max_iter; tight tolerance needs more than OSQP's 4000 default
+    prob = osqp_port_lib.OSQP()
+    prob.setup(P, c["q"], A, c["l"], c["u"], **dict(kw, max_iter=200000))
+    prob.solve()
+    cfg = pendulum(); (nx, nu), Np = cfg["Bd"].shape, cfg["Np"]
+    for t in range(5):
+        prob.update(l=c["upd_l"][t], u=c["upd_u"][t], q=c["upd_q"][t])
+        res = prob.solve()
+        assert res.info.status == "solved"
+        u = res.x[(Np + 1) * nx:(Np + 1) * nx + nu]
+        assert np.max(np.abs(u - g["u"][t])) < 1e-6
 
 
 def test_batch_cpu_driver_matches_single(osqp_port_lib):

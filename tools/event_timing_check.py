@@ -1,5 +1,5 @@
 import sys, os, numpy as np, torch
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from bench import pendulum_batch, make_controller
 B = 65536
 cfg, X0, Xref = pendulum_batch(B, "identical")
